@@ -6,10 +6,13 @@ M=65536, N=512, d=1024, H=8, B=8, on 1/2/4/8 B200 with the key axis M sharded ac
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29511 bench.py --gpus 8 --steps 20 --warmup 5                  # M-sharded
     python bench.py --impl reference --steps 3 --warmup 1              # CPU restatement of the reference
+    python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs out/  # + the last step's output as out/*.npy
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over the synthetic batch:
   value : core attention (QK^T -> softmax -> PV [+ cross-GPU merge]) with q/k/v already resident in
           HBM, timed with CUDA events over exactly K steps, max over ranks.  TFLOP/s = 4*B*N*M*d / t.
+          Inputs are drawn from fixed seeds, so runs with the same arguments see the same q/k/v; --dump-outputs DIR
+          writes what the last of the K steps returned as DIR/attention_out.npy (float32, (B, N, d)) to compare builds.
   e2e   : the same metric through the reference-facing call — ``CrossAttention.forward`` (LayerNorm,
           q/k/v/o projections, attention) — with x_q / x_kv in pinned HOST memory, host->device copies
           and the device->host read of the result inside the timed region.
@@ -26,6 +29,9 @@ import subprocess
 import sys
 import threading
 import time
+
+# the benchmark runs from a tree that may be read-only: leave no bytecode caches in it
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -330,23 +336,32 @@ def run_ours(args, rank, world, local_rank):
             return sharded_attention(q_loc, k, v, H, scale, M, m0, merge=args.merge, copy_out=False, group=mgroup)
 
     def timed(fn, steps, warmup):
+        """-> (ms per step, what the last step returned)."""
         for _ in range(warmup):
             fn()
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1)) / steps
+        return max_over_ranks(e0.elapsed_time(e1)) / steps, last
 
     # ---- value: device-resident core, exactly K steps -------------------------------------------
     launches0 = _lib.launch_count()
     with ClockSampler(local_rank) as clocks:
-        ms_core = timed(core_step, args.steps, args.warmup)
+        ms_core, core_out = timed(core_step, args.steps, args.warmup)
     launches_timed = (_lib.launch_count() - launches0) * args.steps // (args.steps + args.warmup)
     clk = clocks.summary()
+    if args.dump_outputs:
+        import numpy as np
+
+        # the caller's (B, N, d) result of the last timed step, all of it: 16 MiB as float32 at the headline shape
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "attention_out" if world == 1 else f"attention_out.rank{rank}"
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), core_out.float().cpu().numpy())
+    del core_out
 
     # ---- roofline: the dominant kernel alone, events inside the library -----------------------------
     barrier()
@@ -413,8 +428,8 @@ def run_ours(args, rank, world, local_rank):
                 o = cross_attention_sharded(layer, xq, xkv, M, m0, merge=args.merge, group=mgroup).last_hidden_state
         out_host.copy_(o, non_blocking=True)
 
-    e2e_steps = max(1, min(args.steps, args.e2e_steps))
-    ms_e2e = timed(e2e_step, e2e_steps, min(args.warmup, 3))
+    e2e_steps = args.e2e_steps or args.steps
+    ms_e2e, _ = timed(e2e_step, e2e_steps, min(args.warmup, 3))
     h2d = xq_host.numel() * 2 + xkv_host.numel() * 2
     d2h = out_host.numel() * 2
 
@@ -432,7 +447,7 @@ def run_ours(args, rank, world, local_rank):
                 return layer(xq_dev, xkv_dev).last_hidden_state
 
         l0 = _lib.launch_count()
-        ms_mod = timed(module_step, args.steps, min(args.warmup, 3))
+        ms_mod, _ = timed(module_step, args.steps, min(args.warmup, 3))
         l_mod = (_lib.launch_count() - l0) // (args.steps + min(args.warmup, 3))
         mod_flops = flops + 4.0 * B * M * d * d + 4.0 * B * N * d * d
         mod_tf = mod_flops / (ms_mod * 1e-3) / 1e12
@@ -454,12 +469,13 @@ def run_ours(args, rank, world, local_rank):
         del po
         if ops.attention_backward(q, k, v, out_t, go, pm, pl, H, scale, check_only=True):
             l0 = _lib.launch_count()
-            ms_bwd = timed(lambda: ops.attention_backward(q, k, v, out_t, go, pm, pl, H, scale), args.steps,
-                           min(args.warmup, 3))
+            ms_bwd, _ = timed(lambda: ops.attention_backward(q, k, v, out_t, go, pm, pl, H, scale), args.steps,
+                              min(args.warmup, 3))
             l_bwd = (_lib.launch_count() - l0) // (args.steps + min(args.warmup, 3))
-            ms_drop_f = timed(lambda: ops.attention_dropout_forward(q, k, v, pm, pl, H, scale, 0.1, 1234), args.steps, 2)
-            ms_drop_b = timed(lambda: ops.attention_backward(q, k, v, out_t, go, pm, pl, H, scale, dropout_p=0.1,
-                                                             dropout_seed=1234), args.steps, 2)
+            ms_drop_f, _ = timed(lambda: ops.attention_dropout_forward(q, k, v, pm, pl, H, scale, 0.1, 1234),
+                                 args.steps, 2)
+            ms_drop_b, _ = timed(lambda: ops.attention_backward(q, k, v, out_t, go, pm, pl, H, scale, dropout_p=0.1,
+                                                                dropout_seed=1234), args.steps, 2)
             training = {"api": "perceiver_io_b200.ops.attention_backward (pcv_attn_bwd: dK/dV kernel + dQ kernel)",
                         "backward_ms": ms_bwd, "backward_flops": 2.5 * flops,
                         "backward_value": 2.5 * flops / (ms_bwd * 1e-3) / 1e12, "unit": UNIT,
@@ -533,7 +549,7 @@ def main():
     ap.add_argument("--e2e-chunk", type=int, default=8192)
     ap.add_argument("--M", type=int, default=0, help="override the key count (sweep points)")
     ap.add_argument("--B", type=int, default=0)
-    ap.add_argument("--e2e-steps", type=int, default=10)
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the e2e leg (default: --steps)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--decomp", choices=["auto", "m"], default="auto",
@@ -543,7 +559,11 @@ def main():
     ap.add_argument("--skip-training", action="store_true", help="skip the backward / dropout leg")
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes/launch of the dominant kernel from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step of the headline leg as DIR/attention_out.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.e2e_steps < 0:
+        ap.error("--steps must be >= 1 and --e2e-steps >= 0")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

@@ -167,7 +167,8 @@ def layer_cases(core):
                       full_logits=full.logits.clone(), full_hidden=full.last_hidden_state.clone(),
                       full_cache=[(k.clone(), v.clone()) for k, v in full.kv_cache],
                       step_logits=steps, nocache_logits=nocache.logits.clone())
-    torch.save(out, os.path.join(OUT, "layer_cases.pt"))
+    for key, case in out.items():   # one file per case keeps every fixture under 1 MB
+        torch.save(case, os.path.join(OUT, f"layer_{key}.pt"))
     return len(out)
 
 
@@ -235,7 +236,8 @@ def big_cases(core):
             y = m(x_q, x_kv, pad_mask=pad).last_hidden_state
         out[name] = dict(rows=y[:, :: GB.ROW_STEP].clone(), checksums=GB.checksums(sd_, x_q, x_kv),
                          out_abs_max=y.abs().max().item())
-    torch.save(out, os.path.join(OUT, "big_cases.pt"))
+    for name, case in out.items():
+        torch.save(case, os.path.join(OUT, f"big_{name}.pt"))
     return len(out)
 
 

@@ -1,7 +1,7 @@
 """Large reference goldens without large files: the CrossAttention weights and inputs of each case are REBUILT from a
 seed (torch CPU generator — the GPU box runs the same torch build as the authoring container; a float64 checksum of
 every regenerated tensor is stored in the fixture and verified), and only a subsample of the reference's output rows
-is committed (tests/golden/big_cases.pt, written by oracle/gen_golden.py from the REAL reference).
+is committed (tests/golden/big_<case>.pt, written by oracle/gen_golden.py from the REAL reference).
 
 Shapes reach the multi-tile tcgen05 paths the small fixtures never touch: the north-star head geometry
 (C=1024, H=8, dh=128/128) with M=2304 keys and padding, the MLM geometry (32/160), and the optical-flow

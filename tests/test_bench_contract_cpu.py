@@ -24,6 +24,12 @@ def test_reference_arm_prints_one_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=300, cwd=ROOT)
+    assert r.returncode == 2 and "--steps must be >= 1" in r.stderr
+
+
 def test_our_arm_refuses_to_run_without_a_gpu():
     import torch
 

@@ -5,6 +5,7 @@ tolerances are relative to the largest reference magnitude and stated per test."
 import pytest
 import torch
 
+import golden_big as GB
 from conftest import load_golden
 from gpu_util import assert_close, derived_bound, torch_cross_attention
 
@@ -55,7 +56,7 @@ def test_multi_head_attention_golden(case, impl):
         assert out.kv_cache is None
 
 
-LAYERS = load_golden("layer_cases.pt")
+LAYERS = {k: load_golden(f"layer_{k}.pt") for k in ("sab", "cal", "dec", "csm")}
 
 
 def test_self_attention_block_golden():
@@ -231,7 +232,7 @@ def test_streamed_host_input_matches_plain_forward():
 # --------------------------------------------------------------------------------------------------
 # large reference goldens (multi-tile tcgen05 paths) and the training-mode prefix dropout
 # --------------------------------------------------------------------------------------------------
-BIG = load_golden("big_cases.pt")
+BIG = {name: load_golden(f"big_{name}.pt") for name in GB.BIG_CASES}
 
 
 @pytest.mark.parametrize("name", sorted(BIG))
@@ -242,7 +243,6 @@ def test_big_reference_cross_attention_golden(name, dtype):
     (big-head kernel).  Inputs/weights are rebuilt from seeds and verified against the fixture's checksums.  The bound
     is the stated gate, derived here: 2 x |eager-bf16 torch restatement - reference| + 1e-3 x max|reference|.
     The bf16 module additionally runs the fused K/V producer (LayerNorm + k_proj + v_proj on tcgen05)."""
-    import golden_big as GB
     import perceiver_io_b200 as P
 
     kw, sd, x_q, x_kv, pad = GB.build(name)

@@ -1,222 +1,131 @@
-"""-m gpu: the REAL reference (krasserm/perceiver-io, installed unmodified into the git-ignored baseline/_ref by
-baseline/install_ref.py, which travels to the GPU box with the snapshot) as a live oracle:
+"""-m gpu: this package's modules against what the REAL reference (krasserm/perceiver-io) computes on the same models
+and inputs, stored in tests/golden/live_cases.pt by oracle/gen_golden_live.py:
 
   ref64  = the reference model itself, .double(), on the GPU              (the fp64 yardstick)
   eager  = the reference model itself, .bfloat16(), on the GPU            (what its own eager code gives in bf16)
-  ours   = perceiver_io_b200.patch() applied to a copy of the bf16 reference model: same Python objects, same
-           parameters, attention + K/V producer swapped for the sm_100a kernels
+  ours   = the same model built from this package's mirror classes (tests/golden_live.py: same parameter tree, same
+           seeded weights, checked by checksum), in bf16 on the sm_100a kernels
 
-and the stated gate  max|ours - ref64| <= 2 * max|eager - ref64| + 1e-3 * max|ref64|  (BASELINE.md §3).
+and the stated gate  max|ours - ref64| <= 2 * max|eager - ref64| + 1e-3 * max|ref64|  (BASELINE.md §3), with both
+maxima of the gate taken over the whole reference output and |ours - ref64| over the stored sample of its elements.
 Also compares against the reference's own CPU fp32 forward (BASELINE.md §3 names it as the baseline arm)."""
-import copy
-import os
-import sys
-
 import pytest
 import torch
 
-from conftest import ROOT
+import golden_live as GL
+from conftest import load_golden
 from gpu_util import derived_bound
 
 pytestmark = pytest.mark.gpu
 
-sys.path.insert(0, os.path.join(ROOT, "baseline"))
-import install_ref  # noqa: E402
-
-if not install_ref.available():
-    pytest.skip("baseline/_ref is empty (run `python baseline/install_ref.py` where /root/reference exists)",
-                allow_module_level=True)
-core = install_ref.import_reference_core()
+LIVE = load_golden("live_cases.pt")
 
 
-def _randomize(module, seed, scale=None):
-    g = torch.Generator().manual_seed(seed)
-    with torch.no_grad():
-        for name, prm in module.named_parameters():
-            if prm.dim() == 1 and ("norm" in name or name.endswith(".0.weight")) and name.endswith("weight"):
-                prm.copy_(1.0 + 0.1 * torch.randn(prm.shape, generator=g))
-            elif prm.dim() == 1:
-                prm.copy_(0.1 * torch.randn(prm.shape, generator=g))
-            else:
-                s = scale if scale is not None else prm.shape[-1] ** -0.5
-                prm.copy_(s * torch.randn(prm.shape, generator=g))
+def _same_weights(model, case):
+    """The mirror rebuild holds exactly the parameters the reference model was evaluated with."""
+    sums = GL.param_sums(model)
+    assert list(sums) == list(case["params"]), "parameter tree differs from the reference's"
+    for name, val in case["params"].items():
+        assert abs(sums[name] - val) <= 1e-9 * max(1.0, abs(val)), f"regenerated {name} differs from the fixture"
 
 
-def _gate(ours, ref64, eager, what):
-    bound, eager_err, ref_max = derived_bound(ref64, eager)
-    err = (ours.double() - ref64.double()).abs().max().item()
-    print(f"[parity] {what}: err {err:.3e} bound {bound:.3e} (eager {eager_err:.3e}, max|ref| {ref_max:.3e})")
+def _gate(ours, stored, what):
+    """`stored`: a sampled reference output with its full-tensor gate (oracle/gen_golden_live.py `gated`)."""
+    assert tuple(ours.shape) == stored["shape"], (what, tuple(ours.shape), stored["shape"])
     assert torch.isfinite(ours).all(), what
-    assert err <= bound, f"{what}: err {err:.3e} > derived bound {bound:.3e} (eager {eager_err:.3e}, max|ref| {ref_max:.3e})"
+    bound = 2.0 * stored["eager_err"] + 1e-3 * max(stored["ref_max"], 1e-30)
+    err = (GL.sample(ours) - stored["ref"].double()).abs().max().item()
+    print(f"[parity] {what}: err {err:.3e} bound {bound:.3e} (eager {stored['eager_err']:.3e}, "
+          f"max|ref| {stored['ref_max']:.3e})")
+    assert err <= bound, f"{what}: err {err:.3e} > derived bound {bound:.3e} (eager {stored['eager_err']:.3e}, max|ref| {stored['ref_max']:.3e})"
     return err, bound
 
 
-def _patched_bf16(model):
-    import perceiver_io_b200 as P
+def _gate_whole(ours, ref64, eager, what):
+    bound, eager_err, ref_max = derived_bound(ref64, eager)
+    err = (ours.double().cpu() - ref64.double()).abs().max().item()
+    print(f"[parity] {what}: err {err:.3e} bound {bound:.3e} (eager {eager_err:.3e}, max|ref| {ref_max:.3e})")
+    assert torch.isfinite(ours).all(), what
+    assert err <= bound, f"{what}: err {err:.3e} > derived bound {bound:.3e} (eager {eager_err:.3e}, max|ref| {ref_max:.3e})"
 
-    m = copy.deepcopy(model).bfloat16().cuda().eval()
-    n = P.patch(m)
-    assert n > 0
-    return m
 
-
-def test_patch_on_reference_cross_attention_north_star_geometry():
-    import perceiver_io_b200 as P  # noqa: F401
-
-    torch.manual_seed(0)
-    B, N, M, D, H = 2, 384, 2304, 1024, 8
-    ref = core.CrossAttention(num_heads=H, num_q_input_channels=D, num_kv_input_channels=D).eval()
-    _randomize(ref, 1)
+def test_cross_attention_north_star_geometry_matches_reference():
+    case = LIVE["cross_attention"]
+    m, x_q, x_kv, pad = GL.cross_attention(GL.mirror())
+    _same_weights(m, case)
+    mine = m.bfloat16().cuda().eval()
     with torch.no_grad():
-        ref.attention.q_proj.weight.mul_(3.0)   # peaked rows as well
-    g = torch.Generator().manual_seed(2)
-    x_q = torch.randn(1, N, D, generator=g)
-    x_kv = torch.randn(B, M, D, generator=g) + 0.25
-    pad = torch.zeros(B, M, dtype=torch.bool)
-    pad[0, :333] = True
-    pad[1, 2000:] = True
-    xq16, xkv16 = x_q.bfloat16(), x_kv.bfloat16()
-    with torch.no_grad():
-        # every arm sees the same bf16-rounded inputs
-        r64 = copy.deepcopy(ref).double().cuda()(xq16.double().cuda(), xkv16.double().cuda(), pad_mask=pad.cuda()).last_hidden_state
-        eager = copy.deepcopy(ref).bfloat16().cuda()(xq16.cuda(), xkv16.cuda(), pad_mask=pad.cuda()).last_hidden_state
-        mine = _patched_bf16(ref)
-        ours = mine(xq16.cuda(), xkv16.cuda(), pad_mask=pad.cuda()).last_hidden_state
-        assert "_pcv_kv_fold" in mine.__dict__, "patched reference CrossAttention did not take the fused K/V producer"
-        _gate(ours, r64, eager, "reference CrossAttention, patched")
-        # the reference's own CPU fp32 forward (the baseline arm of BASELINE.md §3) on the same rounded inputs
-        cpu = ref(xq16.float(), xkv16.float(), pad_mask=pad).last_hidden_state
-    _gate(ours.cpu(), cpu, eager.cpu(), "vs the reference CPU fp32 forward")
+        ours = mine(x_q.cuda(), x_kv.cuda(), pad_mask=pad.cuda()).last_hidden_state
+    assert "_pcv_kv_fold" in mine.__dict__, "CrossAttention did not take the fused K/V producer"
+    _gate(ours, case["ref64"], "reference CrossAttention")
+    # the reference's own CPU fp32 forward (the baseline arm of BASELINE.md §3) on the same rounded inputs
+    _gate(ours.cpu(), case["cpu"], "vs the reference CPU fp32 forward")
 
 
-class _PassThroughInput(core.InputAdapter):
-    def forward(self, x):
-        return x
+def test_perceiver_encoder_matches_reference():
+    case = LIVE["encoder"]
+    enc, x, pad = GL.encoder(GL.mirror())
+    _same_weights(enc, case)
+    from perceiver_io_b200 import modules
 
-
-def test_patch_on_reference_perceiver_encoder():
-    torch.manual_seed(0)
-    B, M, C, N, D = 2, 3000, 256, 320, 512
-    enc = core.PerceiverEncoder(
-        _PassThroughInput(C), num_latents=N, num_latent_channels=D, num_cross_attention_heads=4,
-        num_cross_attention_layers=2, first_cross_attention_layer_shared=False, num_self_attention_heads=8,
-        num_self_attention_layers_per_block=2, num_self_attention_blocks=2, first_self_attention_block_shared=True,
-        num_cross_attention_qk_channels=256, num_cross_attention_v_channels=512).eval()
-    _randomize(enc, 5)
-    g = torch.Generator().manual_seed(6)
-    x = (torch.randn(B, M, C, generator=g) + 0.1).bfloat16()
-    pad = torch.zeros(B, M, dtype=torch.bool)
-    pad[1, 2500:] = True
-    with torch.no_grad():
-        r64 = copy.deepcopy(enc).double().cuda()(x.double().cuda(), pad_mask=pad.cuda())
-        eager = copy.deepcopy(enc).bfloat16().cuda()(x.cuda(), pad_mask=pad.cuda())
-        from perceiver_io_b200 import modules
-
-        mine = _patched_bf16(enc)
-        modules.kv_producer_config["min_rows_latent"] = 512   # exercise the one-GEMM QKV projection on the 640 latent rows
-        try:
+    mine = enc.bfloat16().cuda().eval()
+    modules.kv_producer_config["min_rows_latent"] = 512   # exercise the one-GEMM QKV projection on the 640 latent rows
+    try:
+        with torch.no_grad():
             ours = mine(x.cuda(), pad_mask=pad.cuda())
-        finally:
-            modules.kv_producer_config["min_rows_latent"] = 4096
+    finally:
+        modules.kv_producer_config["min_rows_latent"] = 4096
     folded = [k for m in mine.modules() for k in m.__dict__ if k.startswith("_pcv_") and k.endswith("_fold")]
     assert "_pcv_qkv_fold" in folded and "_pcv_kv_fold" in folded and "_pcv_o_fold" in folded, folded
-    _gate(ours, r64, eager, "reference PerceiverEncoder, patched (2 cross-attention + 4 self-attention layers)")
+    _gate(ours, case["ref64"], "reference PerceiverEncoder (2 cross-attention + 4 self-attention layers)")
 
 
-def _csm(seed=7):
-    cfg = core.CausalSequenceModelConfig(vocab_size=262, max_seq_len=1536, max_latents=512, num_channels=512, num_heads=8,
-                                         num_self_attention_layers=3, num_self_attention_rotary_layers=1,
-                                         cross_attention_dropout=0.0, output_norm=True, abs_pos_emb=False, init_scale=0.05)
-    m = core.CausalSequenceModel(cfg).eval()
-    _randomize(m, seed, scale=0.04)
-    return m
-
-
-def test_patch_on_reference_causal_sequence_model_logits_and_cache():
+def test_causal_sequence_model_logits_and_cache_match_reference():
     """Perceiver AR: left padding, right-aligned rotary over all head channels, causal prefix cross-attention,
-    causal latent stack; then 3 cached decode steps must agree with the uncached forward (the reference's own
-    tests/kv_cache_test.py:191-234 pattern) and with the reference's fp64 logits.  The bf16 arms run the fp32 model
-    under torch.autocast (Lightning's precision="bf16"): a `.bfloat16()` model computes its rotary angles
-    position x inv_freq in bf16 — radians of error at position 1400 in BOTH arms, which would drown the comparison."""
-    import perceiver_io_b200 as P
-
-    m = _csm()
-    g = torch.Generator().manual_seed(8)
-    B, n0, prefix = 2, 1400, 1000
-    tokens = torch.randint(0, 262, (B, n0 + 3), generator=g)
-    pad = torch.zeros(B, n0 + 3, dtype=torch.bool)
-    pad[1, :57] = True
-    t, p = tokens.cuda(), pad.cuda()
-    with torch.no_grad():
-        m64 = copy.deepcopy(m).double().cuda()
-        m16 = copy.deepcopy(m).cuda()
-        mine = copy.deepcopy(m).cuda()
-        assert P.patch(mine) > 0
-        r64 = m64(t[:, :n0], prefix_len=prefix, pad_mask=p[:, :n0]).logits
+    causal latent stack; then 3 cached decode steps must agree with the reference's uncached forward (the reference's
+    own tests/kv_cache_test.py:191-234 pattern), fp64 and eager.  The bf16 arms run the fp32 model under torch.autocast
+    (Lightning's precision="bf16"): a `.bfloat16()` model computes its rotary angles position x inv_freq in bf16 —
+    radians of error at position 1400 in BOTH arms, which would drown the comparison."""
+    case = LIVE["causal_sequence_model"]
+    m = GL.causal_sequence_model(GL.mirror())
+    _same_weights(m, case)
+    tokens, pad = GL.causal_sequence_tokens()
+    t, p, n0, prefix = tokens.cuda(), pad.cuda(), GL.CSM_N0, GL.CSM_PREFIX
+    mine = m.cuda()
     with torch.no_grad(), torch.autocast("cuda", dtype=torch.bfloat16):
-        eager = m16(t[:, :n0], prefix_len=prefix, pad_mask=p[:, :n0]).logits
         full = mine(t[:, :n0], prefix_len=prefix, pad_mask=p[:, :n0], kv_cache=[])
-        _gate(full.logits, r64, eager, "reference CausalSequenceModel, patched: full forward logits")
+        _gate(full.logits, case["ref64"], "reference CausalSequenceModel: full forward logits")
         cache = full.kv_cache
-        with torch.autocast("cuda", enabled=False):
-            r64_all = m64(t, prefix_len=prefix, pad_mask=p).logits
-        eager_all = m16(t, prefix_len=prefix, pad_mask=p).logits
         for s in range(3):
             step = mine(t[:, n0 + s: n0 + s + 1], prefix_len=prefix, pad_mask=p[:, : n0 + s + 1], kv_cache=cache)
             cache = step.kv_cache
-            # latent n0 - prefix + s of the uncached forward over n0 + 3 tokens
-            j = n0 - prefix + s
-            _gate(step.logits[:, 0], r64_all[:, j], eager_all[:, j], f"cached decode step {s}")
+            _gate_whole(step.logits[:, 0], case["steps"][s]["ref64"], case["steps"][s]["eager"], f"cached decode step {s}")
         assert cache[0][0].shape[1] == n0 + 3 and len(cache) == 1 + 3
 
 
 def test_training_gradients_reach_q_and_k_projections_through_rotary():
-    """ADVICE r1 (high): rotated q / k must stay in the autograd graph.  Patched reference CausalSequenceModel (fp32
-    weights, training mode, no dropout) against the reference's own autograd on the GPU: gradients of the
-    cross-attention and first self-attention layer's q_proj / k_proj weights."""
-    import perceiver_io_b200 as P
-
-    cfg = core.CausalSequenceModelConfig(vocab_size=64, max_seq_len=192, max_latents=64, num_channels=128, num_heads=4,
-                                         num_self_attention_layers=2, num_self_attention_rotary_layers=1,
-                                         cross_attention_dropout=0.0, output_norm=True, abs_pos_emb=False, init_scale=0.05)
-    ref = core.CausalSequenceModel(cfg)
-    _randomize(ref, 11, scale=0.06)
-    ref = ref.cuda().train()
-    mine = copy.deepcopy(ref)
-    assert P.patch(mine) > 0
-    g = torch.Generator().manual_seed(12)
-    tokens = torch.randint(0, 64, (2, 160), generator=g).cuda()
-    pad = torch.zeros(2, 160, dtype=torch.bool)
-    pad[1, :9] = True
-    target = torch.randint(0, 64, (2, 64), generator=g).cuda()
-
-    def grads(model):
-        model.zero_grad()
-        logits = model(tokens, prefix_len=96, pad_mask=pad.cuda()).logits
-        torch.nn.functional.cross_entropy(logits.reshape(-1, 64), target.reshape(-1)).backward()
-        names = ["cross_attention.0.module.attention.q_proj.weight", "cross_attention.0.module.attention.k_proj.weight",
-                 "self_attention.0.0.module.attention.q_proj.weight", "self_attention.0.0.module.attention.k_proj.weight",
-                 "self_attention.1.0.module.attention.v_proj.weight"]
-        prm = dict(model.named_parameters())
-        return {n: prm[n].grad.detach().clone() for n in names}
-
-    gr, gm = grads(ref), grads(mine)
-    for n in gr:
+    """ADVICE r1 (high): rotated q / k must stay in the autograd graph.  CausalSequenceModel (fp32 weights, training
+    mode, no dropout) against the reference's own autograd on the GPU: gradients of the cross-attention and first
+    self-attention layer's q_proj / k_proj weights."""
+    case = LIVE["gradients"]
+    m, tokens, pad, target = GL.gradient_model(GL.mirror())
+    _same_weights(m, case)
+    gm = GL.gradients(m.cuda(), tokens.cuda(), pad.cuda(), target.cuda())
+    for n, ref in case["grads"].items():
         assert gm[n] is not None and gm[n].abs().max().item() > 0, f"no gradient reached {n}"
-        err = (gm[n] - gr[n]).abs().max().item()
-        scale = gr[n].abs().max().item()
+        assert tuple(gm[n].shape) == ref["shape"], n
+        err = (GL.sample(gm[n], GL.GRAD_SAMPLE) - ref["ref"].double()).abs().max().item()
         # forward runs the bf16 tensor-core kernel, backward the torch recompute shim in fp32: bf16 rounding of
         # q/k/v/P (2^-8 each) is the only difference to the reference's fp32 autograd
-        assert err <= 3e-2 * scale, f"{n}: grad err {err:.3e} vs max {scale:.3e}"
+        assert err <= 3e-2 * ref["abs_max"], f"{n}: grad err {err:.3e} vs max {ref['abs_max']:.3e}"
 
 
 def test_cached_generation_under_autocast_promotes_like_torch_cat():
     """ADVICE r1 (medium): under torch.autocast the first cached step meets an fp32 empty cache and bf16 k/v; the
     reference's torch.cat promotes, kv_append must not raise."""
-    import perceiver_io_b200 as P
-
-    m = _csm(3).cuda()
-    assert P.patch(m) > 0
+    m = GL.causal_sequence_model(GL.mirror(), seed=3)
+    _same_weights(m, LIVE["causal_sequence_model_seed3"])
+    m = m.cuda()
     t = torch.randint(0, 262, (1, 300)).cuda()
     with torch.no_grad(), torch.autocast("cuda", dtype=torch.bfloat16):
         full = m(t[:, :299], prefix_len=100, kv_cache=[])
@@ -224,25 +133,17 @@ def test_cached_generation_under_autocast_promotes_like_torch_cat():
     assert torch.isfinite(step.logits).all() and step.kv_cache[0][0].shape[1] == 300
 
 
-def test_patched_reference_encoder_trains_with_attention_dropout():
-    """A real reference PerceiverEncoder built with dropout=0.1, patched, in TRAINING mode: the attention-probability
-    dropout of modules.py:161 runs inside the kernels (round 1 raised here).  Checks: reproducible under
-    torch.manual_seed, differs from the eval forward, mean over seeds approaches it, loss.backward() reaches the input
-    and every parameter through the backward kernels (impl='kernel' raises otherwise), eval is untouched."""
+def test_encoder_trains_with_attention_dropout():
+    """A PerceiverEncoder built with dropout=0.1, in TRAINING mode: the attention-probability dropout of the reference's
+    modules.py:161 runs inside the kernels (round 1 raised here).  Checks: reproducible under torch.manual_seed, differs
+    from the eval forward, mean over seeds approaches it, loss.backward() reaches the input and every parameter through
+    the backward kernels (impl='kernel' raises otherwise), eval is untouched."""
     from perceiver_io_b200 import ops
 
-    torch.manual_seed(0)
-    B, M, C, N, D = 2, 1500, 256, 192, 256
-    enc = core.PerceiverEncoder(
-        _PassThroughInput(C), num_latents=N, num_latent_channels=D, num_cross_attention_heads=4,
-        num_cross_attention_layers=1, num_self_attention_heads=4, num_self_attention_layers_per_block=2,
-        num_self_attention_blocks=1, dropout=0.1)
-    _randomize(enc, 21)
-    mine = _patched_bf16(enc)
-    x = (torch.randn(B, M, C, generator=torch.Generator().manual_seed(22)) + 0.1).bfloat16().cuda()
-    pad = torch.zeros(B, M, dtype=torch.bool)
-    pad[1, 1200:] = True
-    pad = pad.cuda()
+    enc, x, pad = GL.dropout_encoder(GL.mirror())
+    _same_weights(enc, LIVE["dropout_encoder"])
+    mine = enc.bfloat16().cuda()
+    x, pad = x.cuda(), pad.cuda()
     mine.eval()
     with torch.no_grad():
         ev = mine(x, pad_mask=pad).float()

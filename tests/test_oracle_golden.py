@@ -6,6 +6,7 @@ only; the reference's own cache self-consistency bar is 1e-6, tests/kv_cache_tes
 import pytest
 import torch
 
+import golden_big as GB
 from conftest import load_golden
 from oracle import mha_oracle as O
 
@@ -51,7 +52,7 @@ def test_fully_padded_row_is_uniform_average():
     close(case["out"][1], expect)
 
 
-LAYERS = load_golden("layer_cases.pt")
+LAYERS = {k: load_golden(f"layer_{k}.pt") for k in ("sab", "cal", "dec", "csm")}
 
 
 def test_self_attention_block():
@@ -170,15 +171,13 @@ def test_prefix_dropout_integer_path_and_forward():
     close(logits, g["logits"])
 
 
-BIG = load_golden("big_cases.pt")
+BIG = {name: load_golden(f"big_{name}.pt") for name in GB.BIG_CASES}
 
 
 @pytest.mark.parametrize("name", sorted(BIG))
 def test_big_reference_cases_rebuild_and_match_the_oracle(name):
     """The seeded rebuild of weights / inputs reproduces the tensors the fixture was generated from (checksums), and
     the oracle's CrossAttention restatement matches the reference's committed output rows at multi-tile sizes."""
-    import golden_big as GB
-
     kw, sd, x_q, x_kv, pad = GB.build(name)
     sums = GB.checksums(sd, x_q, x_kv)
     for key, val in BIG[name]["checksums"].items():
