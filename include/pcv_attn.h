@@ -307,7 +307,7 @@ typedef struct pcv_shard_fuse {
  * with the masks of the forward (finite fill: a filled score carries no gradient).  Tensors are laid out as in
  * pcv_attn_params ((B, rows, H, d) by strides, in `dtype`); q_stride_b == 0 broadcasts one latent array over the batch and
  * grad_q is then the SUM over the batch, shape (1, N, H*dqk).  Two tcgen05 kernels (dK/dV: key-tile outer; dQ: query-tile
- * outer) — no (B, H, N, M) tensor is ever materialised.  Head dims: multiples of 8, at most 128.
+ * outer; channel-sliced above 128) — no (B, H, N, M) tensor is ever materialised.  Head dims: multiples of 8, at most 512.
  */
 typedef struct pcv_attn_bwd_params {
   const void* q;
@@ -381,7 +381,7 @@ PCV_API int pcv_attn_bwd(const pcv_attn_bwd_params* p, void* stream);
  * probabilities tile by tile, drops each element (b, h, query, key) with probability round(256 p)/256 — a pure function of
  * (dropout_seed, b, h, query, key), regenerated by pcv_attn_bwd from the same seed — scales the survivors by 1/(1 - p) and
  * writes out = dropout(P) V into p->out.  p->workspace must hold pcv_attn_fwd_dropout_workspace_bytes().  Head dims:
- * multiples of 8, at most 128; no key sharding.  pcv_attn_dropout_mask exports the keep mask (B, H, N, M) as bytes
+ * multiples of 8, at most 512; no key sharding.  pcv_attn_dropout_mask exports the keep mask (B, H, N, M) as bytes
  * (tests / debugging).
  */
 PCV_API int pcv_attn_fwd_dropout_supported(const pcv_attn_params* p, float dropout_p);

@@ -108,6 +108,12 @@ int attn_fwd_dropout_workspace_bytes(const pcv_attn_params& p, size_t* bytes);
 int launch_attn_fwd_dropout(const pcv_attn_params& p, const float* stat_m, const float* stat_l, float dropout_p,
                             uint64_t seed, cudaStream_t stream);
 int bwd_debug_read(uint32_t* out, int n);
+// head dims above 128 (pcv_attn_bwd_big.cu); the entry points above route there
+int launch_attn_bwd_big(const pcv_attn_bwd_params& p, cudaStream_t stream);
+int launch_attn_fwd_dropout_big(const pcv_attn_params& p, const float* stat_m, const float* stat_l, float dropout_p,
+                                uint64_t seed, cudaStream_t stream);
+// mapped device pointer of the training kernels' watchdog record (allocated on first use)
+int bwd_diag_record(uint32_t** dptr);
 int launch_dropout_mask(uint8_t* keep, int B, int H, int N, int M, float dropout_p, uint64_t seed, cudaStream_t stream);
 
 }  // namespace pcv

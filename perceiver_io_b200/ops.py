@@ -282,18 +282,33 @@ def dropout_keep_mask(B: int, H: int, N: int, M: int, dropout_p: float, dropout_
     return keep.bool()
 
 
+def _unpad_heads(g: torch.Tensor, shape, num_heads: int) -> torch.Tensor:
+    """(B, L, H*d8) gradient of a ``_pad_heads_to8`` operand -> the original operand's shape (padding channels dropped)."""
+    d = shape[2] // num_heads if len(shape) == 3 else shape[3]
+    return g.reshape(g.shape[0], g.shape[1], num_heads, -1)[..., :d].reshape(shape)
+
+
 class _FusedAttention(torch.autograd.Function):
     """Forward = the fused CUDA kernel (partial-state mode, so the row max and denominator are kept).
     Backward = the tcgen05 backward kernels (``attention_backward`` -> pcv_attn_bwd: dK/dV and dQ kernels, SURVEY.md
-    §8(f) rank 2) for head dims that are multiples of 8 up to 128.  Other shapes take the labelled SHIM below: the
-    flash-attention backward recurrence in plain torch ops, chunked over the key axis from the saved statistics,
-    memory bounded by ``backward_config["max_score_bytes"]``; neither path ever holds the (B, H, N, M) score tensor
-    (8.6 GB at the north-star shape).  The inference forward never routes through this class."""
+    §8(f) rank 2) for head dims up to 512.  Head dims that are not multiples of 8 are zero-padded to the next multiple
+    in the forward (the statistics of the padded problem are those of the original one) and the outputs and gradients
+    sliced back.  Other calls (CPU tensors, ``impl="decode"``) take the labelled SHIM below: the flash-attention
+    backward recurrence in plain torch ops, chunked over the key axis from the saved statistics, memory bounded by
+    ``backward_config["max_score_bytes"]``; neither path ever holds the (B, H, N, M) score tensor (8.6 GB at the
+    north-star shape).  The inference forward never routes through this class."""
 
     @staticmethod
     def forward(ctx, q, k, v, num_heads, scale, pad_mask, causal, impl, dropout_p=0.0, dropout_seed=0):
         dv_true = _head_dim(v, num_heads)
         ctx.dropout = (float(dropout_p), int(dropout_seed))
+        ctx.padded_from = None
+        if impl != "decode" and (_head_dim(q, num_heads) % 8 or dv_true % 8):
+            # pad to multiples of 8 so that the partial-state kernels take the call and their statistics are saved;
+            # zero channels change neither q.k nor the first dv channels of P.V, and the gradient of a zero channel
+            # is dropped when the gradients are sliced back (backward)
+            ctx.padded_from = (tuple(q.shape), tuple(k.shape), tuple(v.shape))
+            q, k, v = (_pad_heads_to8(t, num_heads).flatten(2) for t in (q, k, v))
         if dropout_p > 0.0:
             # statistics from the fused kernel, then the dropout pass (second kernel) writes the output
             po, pm, pl = attention_partial(q, k, v, num_heads, scale, pad_mask=pad_mask, causal=causal, impl=impl)
@@ -301,9 +316,7 @@ class _FusedAttention(torch.autograd.Function):
             out = attention_dropout_forward(q, k, v, pm, pl, num_heads, scale, dropout_p, dropout_seed, pad_mask, causal)
             out = out if out.dtype == q.dtype else out.to(q.dtype)
             ctx.save_for_backward(q, k, v, pad_mask, out, pm, pl)
-            ctx.meta = (num_heads, scale, causal)
-            return out
-        if _head_dim(q, num_heads) % 8 or dv_true % 8 or impl == "decode":
+        elif _head_dim(q, num_heads) % 8 or _head_dim(v, num_heads) % 8 or impl == "decode":
             # head dims the partial-state kernels do not take without padding: plain forward, statistics recomputed
             out = _attention_forward(q, k, v, num_heads, scale, pad_mask, causal, impl)
             ctx.save_for_backward(q, k, v, pad_mask, out, None, None)
@@ -313,10 +326,24 @@ class _FusedAttention(torch.autograd.Function):
             out = out if out.dtype == q.dtype else out.to(q.dtype)
             ctx.save_for_backward(q, k, v, pad_mask, out, pm, pl)
         ctx.meta = (num_heads, scale, causal)
+        if ctx.padded_from is not None:
+            out = out.reshape(out.shape[0], out.shape[1], num_heads, -1)[..., :dv_true].flatten(2)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
+        padded_from = getattr(ctx, "padded_from", None)
+        H = ctx.meta[0]
+        if padded_from is not None:
+            grad_out = _pad_heads_to8(grad_out, H).flatten(2)
+        gq, gk, gv = _FusedAttention._grads(ctx, grad_out)
+        if padded_from is not None:
+            gq, gk, gv = (_unpad_heads(g, shape, H) for g, shape in zip((gq, gk, gv), padded_from))
+        return gq, gk, gv, None, None, None, None, None, None, None
+
+    @staticmethod
+    def _grads(ctx, grad_out):
+        """(grad_q, grad_k, grad_v) of the saved (padded) operands: the kernels, or the shim."""
         q, k, v, pad_mask, out, pm, pl = ctx.saved_tensors
         H, scale, causal = ctx.meta
         drop_p, drop_seed = getattr(ctx, "dropout", (0.0, 0))
@@ -330,7 +357,7 @@ class _FusedAttention(torch.autograd.Function):
             if ok:
                 gq, gk, gv = attention_backward(q, k, v, out, grad_out, pm, pl, H, scale, pad_mask, causal,
                                                 dropout_p=drop_p, dropout_seed=drop_seed)
-                return gq.to(q.dtype), gk.to(k.dtype), gv.to(v.dtype), None, None, None, None, None, None, None
+                return gq.to(q.dtype), gk.to(k.dtype), gv.to(v.dtype)
             if mode == "kernel":
                 raise RuntimeError("backward_config['impl'] = 'kernel' but pcv_attn_bwd does not cover this call: "
                                    + _lib.lib().pcv_last_error().decode())
@@ -392,7 +419,7 @@ class _FusedAttention(torch.autograd.Function):
             gq = gq.sum(0, keepdim=True)
         gk = (gk * scale).transpose(1, 2).reshape(B, M, -1)
         gv = gv.transpose(1, 2).reshape(B, M, -1)
-        return gq.to(q.dtype), gk.to(k.dtype), gv.to(v.dtype), None, None, None, None, None, None, None
+        return gq.to(q.dtype), gk.to(k.dtype), gv.to(v.dtype)
 
 
 def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, num_heads: int, scale: float,
@@ -405,12 +432,15 @@ def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, num_heads: int,
     (/root/reference/perceiver/model/core/modules.py): q is scaled by ``scale``, ``pad_mask`` (True =
     padding) and the right-aligned causal mask use the finite fill ``-finfo.max``.  ``dropout_p`` > 0 applies the
     reference's dropout on the attention probabilities (:161) with a counter-based mask derived from
-    ``dropout_seed`` (default: a fresh seed from torch's CPU generator); head dims must be multiples of 8 up to 128.
+    ``dropout_seed`` (default: a fresh seed from torch's CPU generator); head dims up to 512 (not multiples of 8: padded).
     """
     if dropout_p > 0.0:
         if not 0.0 < dropout_p < 1.0:
             raise ValueError(f"dropout_p must be in [0, 1), got {dropout_p}")
-        if not attention_dropout_forward(q, k, v, None, None, num_heads, scale, dropout_p, 0, pad_mask, causal,
+        probe = (q, k, v)
+        if _head_dim(q, num_heads) % 8 or _head_dim(v, num_heads) % 8:  # the forward pads these (_FusedAttention)
+            probe = tuple(_pad_heads_to8(t, num_heads).flatten(2) for t in probe)
+        if not attention_dropout_forward(*probe, None, None, num_heads, scale, dropout_p, 0, pad_mask, causal,
                                          check_only=True):
             raise NotImplementedError("attention dropout is not available for this call: "
                                       + _lib.lib().pcv_last_error().decode())
